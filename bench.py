@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps 4 --warmup 3                 # our arm, headline workload 25x4x72x128
     python bench.py --impl reference --steps 2 --warmup 1         # the reference's algorithm on the host CPU cores
+    python bench.py --steps 4 --warmup 3 --dump-outputs DIR       # + the last timed step's x_prev / pred_x0 as DIR/*.npy
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # frame/CFG-sharded, N in {2,4,8}
 
 One "step" = one DDIMSampler.p_sample_ddim: 2 U-Net forwards (cond + uncond, CFG 7.5), guidance rescale 0.7,
@@ -331,7 +332,11 @@ def main():
     ap.add_argument("--no-batch-cfg", action="store_true")
     ap.add_argument("--no-cfg-split", action="store_true", help="N > 1: pure frame sharding (every rank runs the B=2 cond+uncond forward on its frames) instead of 2-way CFG split x N/2-way frames")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from the host instead of replaying the captured forward")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step returned (x_prev, pred_x0) "
+                                                          "as DIR/<name>.npy in float32; the same arguments give the same inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -454,12 +459,14 @@ def main():
     with ClockSampler(local_rank) as clk:
         e0.record()
         for i in range(args.steps):
-            x, _ = run_step(x, args.warmup + i)
+            x, pred_x0 = run_step(x, args.warmup + i)
         e1.record()
         barrier()
     launches = int(lib.vc_launch_count()) + int(unet_m.graph_replayed_launches)   # host-launched + executed through graph replays
     t_dev = torch.tensor([e0.elapsed_time(e1) * 1e-3], device=device, dtype=torch.float64)
     finite = bool(torch.isfinite(x).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x_prev=x, pred_x0=pred_x0)
 
     # ---- end to end through the sampler API with HOST buffers: H2D of the step inputs + D2H of x_{t-1} every step ----
     # The sampler API takes the conditioning once per clip (ddim.py:61-134 / utils/diffusion_utils.py:117-201), so it stays
@@ -542,6 +549,14 @@ def main():
             line["cpu_baseline_config1"] = cpu_config1_measured(sd_cpu)
     print(json.dumps(line))
     _finish(world, dist)
+
+
+def dump_outputs(out_dir, **arrays):
+    """What a caller of the timed path received from its last step, one DIR/<name>.npy (float32) per array.  Weights, inputs and
+    the per-step noise all come from fixed seeds, so two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().float().cpu().numpy())
 
 
 def _finish(world, dist):

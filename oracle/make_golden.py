@@ -294,9 +294,70 @@ def gen_resampler():
     print("resampler out std", float(y.std()))
 
 
+DROPIN_CASES = ((False, 16), (True, 16), (False, 5))     # (multiple_cond_cfg, T)
+DROPIN_STRIDE = 17                                       # every 17th output value is stored: ~15k of the 197k at T = 16
+
+
+def gen_dropin():
+    """The reference's own pipeline end to end: its VIPLatentDiffusion from its YAML (configs/inference_pvd_1024.yaml, reduced
+    widths, the two OpenCLIP towers replaced by the toys of oracle/synth.py) and its utils.diffusion_utils.image_guided_synthesis
+    with its own samplers.  T = 16: 77 + 16 T = 333 context tokens -> per-frame image tokens (openaimodel3d.py:556-560); T = 5: the
+    shared-context branch the 25-frame checkpoints take.  Stored: the constructor arguments, the (name, shape) list of the three
+    networks' weights (seed 81), the synthesis arguments and a strided sample of each output with the std of the whole output."""
+    import yaml
+    ref_shims.install()
+    import utils.diffusion_utils as DU
+    import lvdm.models.samplers.ddim as ref_ddim
+    import lvdm.models.samplers.ddim_multiplecond as ref_multi
+
+    def on_cpu(cls):                                      # ddim.py:18-22 hard-codes "cuda"
+        return type("CpuSampler", (cls,), {"register_buffer": lambda self, name, attr: setattr(self, name, attr)})
+
+    DU.DDIMSampler, DU.DDIMSampler_multicond = on_cpu(ref_ddim.DDIMSampler), on_cpu(ref_multi.DDIMSampler)
+    cfg = yaml.safe_load(open(os.path.join(ref_shims.REF_ROOT, "configs", "inference_pvd_1024.yaml")))["model"]
+    P = cfg["params"]
+    P["unet_config"]["params"].update(model_channels=64, use_checkpoint=False)
+    P["first_stage_config"]["params"]["ddconfig"].update(ch=32)
+    P["cond_stage_config"] = {"target": "oracle.synth.ToyText"}
+    P["img_cond_stage_config"] = {"target": "oracle.synth.ToyImage"}
+    P["image_proj_stage_config"]["params"].update(dim=128, depth=1, heads=2, embedding_dim=64)      # still 16 x 16 queries -> 1024
+
+    class _AD(dict):                                      # OmegaConf's attribute access, as instantiate_from_config reads it
+        __getattr__ = dict.__getitem__
+
+    def ad(x):
+        return _AD({k: ad(v) for k, v in x.items()}) if isinstance(x, dict) else [ad(v) for v in x] if isinstance(x, list) else x
+
+    torch.manual_seed(0)
+    ref = DU.instantiate_from_config(ad(cfg)).eval()
+    nets = ("model.", "first_stage_model.", "image_proj_model.")
+    shapes = [(k, s) for k, s in synth.module_shapes(ref) if k.startswith(nets)]
+    ref.load_state_dict(synth.synth_state_dict(shapes, seed=81), strict=False)
+    out = {"shapes": json.dumps([[n, list(s)] for n, s in shapes]),
+           "unet_config": json.dumps(P["unet_config"]["params"]),
+           "first_stage_config": json.dumps(P["first_stage_config"]["params"]),
+           "image_proj_config": json.dumps(P["image_proj_stage_config"]["params"]),
+           "model_params": json.dumps({k: v for k, v in P.items() if not isinstance(v, dict)}),
+           "stride": np.asarray(DROPIN_STRIDE)}
+    H, W = 8, 8
+    for multi, T in DROPIN_CASES:
+        videos = torch.rand(1, 3, T, 8 * H, 8 * W, generator=torch.Generator().manual_seed(7)) * 2 - 1
+        kw = dict(n_samples=1, ddim_steps=(1 if multi else 2), ddim_eta=1.0, unconditional_guidance_scale=7.5, cfg_img=(2.0 if multi else None),
+                  fs=10, text_input=True, multiple_cond_cfg=multi, timestep_spacing="uniform_trailing", guidance_rescale=0.7, condition_index=[0])
+        torch.manual_seed(11)
+        y = DU.image_guided_synthesis(ref, ["a photo"], videos, [1, 4, T, H, W], **kw)
+        tag = f"multi{int(multi)}_T{T}"
+        out[f"{tag}_kwargs"] = json.dumps(kw)
+        out[f"{tag}_shape"] = np.asarray(y.shape)
+        out[f"{tag}_std"] = np.asarray(float(y.std()))
+        out[f"{tag}_sample"] = y.reshape(-1)[::DROPIN_STRIDE].numpy()
+        print(tag, "out std", float(y.std()), "stored", out[f"{tag}_sample"].size)
+    np.savez_compressed(os.path.join(OUT, "dropin_pipeline.npz"), **out)
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ["schedule", "ddim", "ddim_options", "ddim_multicond", "unet", "vae", "vae_enc", "resampler"]
+    which = sys.argv[1:] or ["schedule", "ddim", "ddim_options", "ddim_multicond", "unet", "vae", "vae_enc", "resampler", "dropin"]
     with torch.no_grad():
         for w in which:
             globals()["gen_" + w]()

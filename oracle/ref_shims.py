@@ -1,7 +1,7 @@
-"""Import the UNMODIFIED reference modules from /root/reference (build container only).
+"""Import the UNMODIFIED reference modules from a checkout of the reference (VC_REFERENCE_ROOT).
 
-TEST INFRASTRUCTURE.  Used by oracle/make_golden.py and by tests that validate the oracle
-against the live reference when /root/reference is present.  Never imported by the product.
+TEST INFRASTRUCTURE.  Used by oracle/make_golden.py to write tests/golden/; the tests only read
+those fixtures.  Never imported by the product.
 
 Shims (SURVEY.md §8c): a stub ``pytorch_lightning`` package (the reference only uses it as a
 base class), and on CPU an override of ``DDIMSampler.register_buffer`` because

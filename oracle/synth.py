@@ -35,3 +35,29 @@ def synth_state_dict(shapes: Iterable[Tuple[str, Tuple[int, ...]]], seed: int = 
 
 def module_shapes(module: torch.nn.Module):
     return [(k, tuple(v.shape)) for k, v in module.state_dict().items()]
+
+
+class ToyText(torch.nn.Module):
+    """Stands in for FrozenOpenCLIPEmbedder (condition.py:174-234): "" and any other prompt map to two fixed 77-token contexts."""
+
+    def __init__(self):
+        super().__init__()
+        self.register_buffer("tab", torch.randn(2, 77, 1024, generator=torch.Generator().manual_seed(5)))
+
+    def forward(self, prompts):
+        return torch.cat([self.tab[0:1] if p == "" else self.tab[1:2] for p in prompts], 0)
+
+    def encode(self, prompts):
+        return self(prompts)
+
+
+class ToyImage(torch.nn.Module):
+    """Stands in for FrozenOpenCLIPImageEmbedderV2 (condition.py:295-372): a fixed projection of a 4x4 pooled image."""
+
+    def __init__(self, tokens=9, dim=64):
+        super().__init__()
+        self.register_buffer("w", torch.randn(48, tokens * dim, generator=torch.Generator().manual_seed(6)) * 0.2)
+        self.tokens, self.dim = tokens, dim
+
+    def forward(self, img):
+        return (torch.nn.functional.adaptive_avg_pool2d(img.float(), 4).flatten(1) @ self.w).reshape(img.shape[0], self.tokens, self.dim)

@@ -1,135 +1,73 @@
-"""The drop-in claim, end to end, against the LIVE reference (build container only; skipped where /root/reference is absent):
+"""The drop-in claim, end to end, against outputs of the UNMODIFIED reference pipeline (tests/golden/dropin_pipeline.npz,
+written by oracle/make_golden.py):
 
-the reference's own ``VIPLatentDiffusion`` is instantiated from its own YAML (configs/inference_pvd_1024.yaml, reduced widths)
-twice -- once untouched, once with the three ``target:`` lines of INTEGRATION.md pointing at viewcrafter_b200 (UNetModel,
-AutoencoderKL, Resampler) -- the SAME state dict is loaded into both with ``strict=True``, and the reference's own
-``utils.diffusion_utils.image_guided_synthesis`` is run on both (reference DDIMSampler vs viewcrafter_b200 DDIMSampler, the
-one-line import swap of INTEGRATION.md).  The CUDA ops are replaced by the torch double, so this checks every seam of the
-boundary (constructor kwargs, state-dict keys, encode/decode types the reference type-checks, kwargs swallowed by forward, RNG
-order), not the kernels.  Shims: SURVEY.md 8(c) -- a pytorch_lightning stub, an attribute dict for OmegaConf, toy stand-ins for
-the two OpenCLIP towers (open_clip / kornia are not installed), and the CPU register_buffer override of the reference sampler.
-T = 16 so that the per-frame image-token context branch (openaimodel3d.py:556-560) is the one exercised.
+the reference ran its own ``VIPLatentDiffusion``, instantiated from its own YAML (configs/inference_pvd_1024.yaml, reduced
+widths), and its own ``utils.diffusion_utils.image_guided_synthesis`` with its own samplers, on weights synthesised from the
+stored (name, shape) list.  Here the U-Net, AutoencoderKL and Resampler of viewcrafter_b200 are built from the constructor
+arguments the YAML gave the reference's classes, must carry the same state-dict keys and shapes in the same order, get the
+same weights, and run through viewcrafter_b200's ``LatentDiffusion`` wrapper, samplers and ``image_guided_synthesis`` with
+the same arguments and seeds.  The CUDA ops are replaced by the torch double, so this checks every seam of the boundary
+(constructor kwargs, state-dict keys, conditioning construction, RNG order, decode), not the kernels.  The two OpenCLIP
+towers are the toys of oracle/synth.py on both sides.  T = 16 so that the per-frame image-token context branch
+(openaimodel3d.py:556-560) is exercised, T = 5 for the shared-context branch of the 25-frame checkpoints.
 """
-import copy
-import sys
-import types
+import json
+import os
 
+import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shims, synth
+from oracle import synth
 from tests import fake_ops
 
-pytestmark = pytest.mark.skipif(not ref_shims.available(), reason="live reference (/root/reference) not present")
+NETS = ("model.", "first_stage_model.", "image_proj_model.")
 
 
-class _AD(dict):
-    __getattr__ = dict.__getitem__
+def _model(gd):
+    from viewcrafter_b200.diffusion import LatentDiffusion
+    from viewcrafter_b200.resampler import Resampler
 
+    class Model(LatentDiffusion):                         # the attribute surface image_guided_synthesis reads (synthesis.py)
+        def __init__(self, P):
+            super().__init__(json.loads(str(gd["unet_config"])), json.loads(str(gd["first_stage_config"])),
+                             **{k: P[k] for k in ("timesteps", "linear_start", "linear_end", "rescale_betas_zero_snr", "parameterization",
+                                                  "scale_factor", "use_dynamic_rescale", "base_scale", "perframe_ae", "conditioning_key")})
+            self.uncond_type = P["uncond_type"]
+            self.cond_stage_model = synth.ToyText()
+            self.embedder = synth.ToyImage()
+            self.image_proj_model = Resampler(**json.loads(str(gd["image_proj_config"])))
 
-def _ad(x):
-    if isinstance(x, dict):
-        return _AD({k: _ad(v) for k, v in x.items()})
-    if isinstance(x, list):
-        return [_ad(v) for v in x]
-    return x
+        def get_learned_conditioning(self, c):
+            return self.cond_stage_model.encode(c)
 
-
-def _toys():
-    if "vc_test_toys" in sys.modules:
-        return
-    m = types.ModuleType("vc_test_toys")
-
-    class ToyText(torch.nn.Module):                      # stands in for FrozenOpenCLIPEmbedder (condition.py:174-234)
-        def __init__(self):
-            super().__init__()
-            self.register_buffer("tab", torch.randn(2, 77, 1024, generator=torch.Generator().manual_seed(5)))
-
-        def forward(self, prompts):
-            return torch.cat([self.tab[0:1] if p == "" else self.tab[1:2] for p in prompts], 0)
-
-        def encode(self, prompts):
-            return self(prompts)
-
-    class ToyImage(torch.nn.Module):                     # stands in for FrozenOpenCLIPImageEmbedderV2 (condition.py:295-372)
-        def __init__(self, tokens=9, dim=64):
-            super().__init__()
-            self.register_buffer("w", torch.randn(48, tokens * dim, generator=torch.Generator().manual_seed(6)) * 0.2)
-            self.tokens, self.dim = tokens, dim
-
-        def forward(self, img):
-            return (torch.nn.functional.adaptive_avg_pool2d(img.float(), 4).flatten(1) @ self.w).reshape(img.shape[0], self.tokens, self.dim)
-
-    m.ToyText, m.ToyImage = ToyText, ToyImage
-    sys.modules["vc_test_toys"] = m
+    torch.manual_seed(0)
+    return Model(json.loads(str(gd["model_params"]))).eval()
 
 
 @pytest.mark.parametrize("multi,T", [(False, 16), (True, 16), (False, 5)])
-def test_reference_pipeline_with_dropins_matches_reference(monkeypatch, multi, T):
-    """T = 16: 77 + 16 T = 333 context tokens -> per-frame image tokens (openaimodel3d.py:556-560); T = 5: the shared-context
-    branch the 25-frame checkpoints take."""
-    import yaml
-    ref_shims.install()
-    _toys()
+def test_reference_pipeline_with_dropins_matches_reference(monkeypatch, golden_dir, multi, T):
+    """T = 16: 77 + 16 T = 333 context tokens -> per-frame image tokens (openaimodel3d.py:556-560); T = 5: the
+    shared-context branch the 25-frame checkpoints take."""
+    from viewcrafter_b200.synthesis import image_guided_synthesis
     fake_ops.install(monkeypatch)
-    import utils.diffusion_utils as DU
-    cfg = yaml.safe_load(open(ref_shims.REF_ROOT + "/configs/inference_pvd_1024.yaml"))["model"]
-    P = cfg["params"]
-    P["unet_config"]["params"].update(model_channels=64, use_checkpoint=False)
-    P["first_stage_config"]["params"]["ddconfig"].update(ch=32)
-    P["cond_stage_config"] = {"target": "vc_test_toys.ToyText"}
-    P["img_cond_stage_config"] = {"target": "vc_test_toys.ToyImage"}
-    P["image_proj_stage_config"]["params"].update(dim=128, depth=1, heads=2, embedding_dim=64)      # still 16 x 16 queries -> 1024
-
-    def build(ours):
-        c = copy.deepcopy(cfg)
-        if ours:                                          # exactly the YAML edit INTEGRATION.md describes
-            c["params"]["unet_config"]["target"] = "viewcrafter_b200.unet.UNetModel"
-            c["params"]["first_stage_config"]["target"] = "viewcrafter_b200.autoencoder.AutoencoderKL"
-            c["params"]["image_proj_stage_config"]["target"] = "viewcrafter_b200.resampler.Resampler"
-        torch.manual_seed(0)
-        return DU.instantiate_from_config(_ad(c)).eval()
-
-    ref = build(False)
-    sd = synth.synth_state_dict(synth.module_shapes(ref), seed=81)
-    for k, v in ref.state_dict().items():                # schedule buffers keep the values the reference computed
-        if not k.startswith(("model.", "first_stage_model.", "image_proj_model.")):
-            sd[k] = v.clone()
-    ref.load_state_dict(sd, strict=True)
-    mine = build(True)
-    assert list(mine.state_dict().keys()) == list(ref.state_dict().keys())
-    mine.load_state_dict(sd, strict=True)                # load_model_checkpoint(..., strict=True), diffusion_utils.py:83-108
+    gd = np.load(os.path.join(golden_dir, "dropin_pipeline.npz"))
+    tag = f"multi{int(multi)}_T{T}"
+    mine = _model(gd)
+    ref_shapes = [(n, tuple(s)) for n, s in json.loads(str(gd["shapes"]))]
+    assert [(k, s) for k, s in synth.module_shapes(mine) if k.startswith(NETS)] == ref_shapes     # names, shapes AND order
+    sd = mine.state_dict()
+    sd.update(synth.synth_state_dict(ref_shapes, seed=81))
+    mine.load_state_dict(sd, strict=True)
 
     H, W = 8, 8
     videos = torch.rand(1, 3, T, 8 * H, 8 * W, generator=torch.Generator().manual_seed(7)) * 2 - 1
-    kw = dict(n_samples=1, ddim_steps=(1 if multi else 2), ddim_eta=1.0, unconditional_guidance_scale=7.5, cfg_img=(2.0 if multi else None),
-              fs=10, text_input=True, multiple_cond_cfg=multi, timestep_spacing="uniform_trailing", guidance_rescale=0.7, condition_index=[0])
-
-    import lvdm.models.samplers.ddim as ref_ddim
-    import lvdm.models.samplers.ddim_multiplecond as ref_multi
-
-    def on_cpu(cls):                                      # ddim.py:18-22 hard-codes "cuda"
-        return type("CpuSampler", (cls,), {"register_buffer": lambda self, name, attr: setattr(self, name, attr)})
-
-    monkeypatch.setattr(DU, "DDIMSampler", on_cpu(ref_ddim.DDIMSampler))
-    monkeypatch.setattr(DU, "DDIMSampler_multicond", on_cpu(ref_multi.DDIMSampler))
+    kw = json.loads(str(gd[f"{tag}_kwargs"]))
     torch.manual_seed(11)
-    with torch.no_grad():
-        out_ref = DU.image_guided_synthesis(ref, ["a photo"], videos, [1, 4, T, H, W], **kw)
-    from viewcrafter_b200.ddim import DDIMSampler
-    from viewcrafter_b200.ddim_multiplecond import DDIMSampler as DDIMSampler_multicond
-    monkeypatch.setattr(DU, "DDIMSampler", DDIMSampler)                      # the import swap of INTEGRATION.md (b)
-    monkeypatch.setattr(DU, "DDIMSampler_multicond", DDIMSampler_multicond)
-    torch.manual_seed(11)
-    with torch.no_grad():
-        out_mine = DU.image_guided_synthesis(mine, ["a photo"], videos, [1, 4, T, H, W], **kw)
-    assert out_mine.shape == out_ref.shape == (1, 1, 3, T, 8 * H, 8 * W) and out_mine.dtype == out_ref.dtype
-    err = (out_mine - out_ref).abs()
-    std = float(out_ref.std())
+    out = image_guided_synthesis(mine, ["a photo"], videos, [1, 4, T, H, W], **kw)
+    assert tuple(out.shape) == tuple(gd[f"{tag}_shape"]) == (1, 1, 3, T, 8 * H, 8 * W) and out.dtype == torch.float32
+    ref = torch.from_numpy(gd[f"{tag}_sample"])
+    err = (out.reshape(-1)[::int(gd["stride"])] - ref).abs()
+    std = float(gd[f"{tag}_std"])
     # fp16 rounding points of the kernels (emulated by the op double) vs the fp32 reference, amplified ~16x by CFG 7.5 per step
     assert float(err.mean()) < 0.03 * std and float(err.max()) < 0.35 * std, (float(err.mean()), float(err.max()), std)
-    # and our own image_guided_synthesis (viewcrafter_b200/synthesis.py) is the same function on the same model
-    from viewcrafter_b200.synthesis import image_guided_synthesis
-    torch.manual_seed(11)
-    out_syn = image_guided_synthesis(mine, ["a photo"], videos, [1, 4, T, H, W], **kw)
-    assert float((out_syn - out_mine).abs().mean()) < 0.02 * std
