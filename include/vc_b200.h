@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define VC_B200_ABI_VERSION 6
+#define VC_B200_ABI_VERSION 7
 
 int vc_abi_version(void);
 const char* vc_last_error(void);
@@ -203,7 +203,7 @@ typedef struct vc_peer_comm {
   void* done;                        /* own uint32: scratch (zero-initialised)                                      */
   void* stats_slots[8];              /* rank p's float[2][Bmax][world][64] as mapped here                           */
   void* cur_stats;                   /* own float[Bmax][world][64]                                                  */
-  int32_t Bmax;                      /* batch samples per rank the slots were sized for (1 or 2)                    */
+  int32_t Bmax;                      /* batch samples per rank the slots were sized for (1..4)                      */
 } vc_peer_comm;
 int vc_enable_peer_access(int32_t peer_device);
 /* IPC-shareable, zero-filled device memory (cudaMalloc) + its 64-byte cudaIpcMemHandle_t; vc_peer_open maps another process's

@@ -10,7 +10,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VC_B200_LIB") or os.path.join(_HERE, "libvc_b200.so")   # override: A/B builds of the kernels
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 
 class VcError(RuntimeError):

@@ -25,6 +25,9 @@
 namespace vc {
 
 static constexpr int PEER_MAX = 8;
+static constexpr int PEER_BMAX = 4;                 // batch samples per rank (vc_peer_comm.Bmax): e.g. the three branches of three-way CFG
+static constexpr int PEER_ALLREDUCE_THREADS = 128;  // gn_peer_allreduce_kernel block (peer_finish loops over the B*64 sums)
+static_assert(PEER_ALLREDUCE_THREADS >= PEER_MAX, "peer_finish: one thread per rank signals / waits");
 
 struct PeerCommDev {
   int world, rank;
@@ -60,15 +63,21 @@ __device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int* p) {
 }
 
 // Tail of every collective, executed by ALL threads of the LAST CTA of this rank (the caller has established that every other
-// CTA's stores are fenced): publish `mine` (B*64 partial sums, or nothing), signal, wait for all peers, gather their sums.
-__device__ __forceinline__ void peer_finish(const PeerCommDev& pc, int B, bool with_stats, float mine, int tid) {
+// CTA's stores are fenced): publish this rank's B*64 partial sums (the sum over `splits` of partial[b][split][64]; nothing when
+// !with_stats), signal, wait for all peers, gather their sums.  Strided over B*64 values, so any block size covers up to PEER_BMAX
+// samples; the signal / wait step needs blockDim.x >= world (checked on the host before every launch).
+__device__ __forceinline__ void peer_finish(const PeerCommDev& pc, int B, bool with_stats, const float* partial, int splits, int tid) {
   const unsigned int s = *reinterpret_cast<volatile unsigned int*>(pc.seq) + 1u;
   const int n = B * 64;
   const int parity = (int)(s & 1u);
-  if (with_stats && tid < n) {
-    const int b = tid >> 6, t = tid & 63;
-    const long long slot = (((long long)parity * pc.Bmax + b) * pc.world + pc.rank) * 64 + t;
-    for (int q = 0; q < pc.world; ++q) pc.stats_slots[q][slot] = mine;
+  if (with_stats) {
+    for (int i = tid; i < n; i += blockDim.x) {
+      const int b = i >> 6, t = i & 63;
+      float mine = 0.f;
+      for (int sp = 0; sp < splits; ++sp) mine += __ldcg(partial + ((long long)b * splits + sp) * 64 + t);
+      const long long slot = (((long long)parity * pc.Bmax + b) * pc.world + pc.rank) * 64 + t;
+      for (int q = 0; q < pc.world; ++q) pc.stats_slots[q][slot] = mine;
+    }
   }
   __threadfence_system();
   __syncthreads();
@@ -180,25 +189,15 @@ __global__ void __launch_bounds__(512) peer_exchange_kernel(const __grid_constan
   }
   __syncthreads();
   if (!is_last) return;
-  float mine = 0.f;
-  if (p.with_stats && tid < p.B * 64) {
-    const int bb = tid >> 6, t = tid & 63;
-    for (int spx = 0; spx < p.splits; ++spx) mine += __ldcg(p.partial + ((long long)bb * p.splits + spx) * 64 + t);
-  }
-  peer_finish(p.pc, p.B, p.with_stats != 0, mine, tid);
+  peer_finish(p.pc, p.B, p.with_stats != 0, p.partial, p.splits, tid);
 }
 
 // (sum, sumsq) per group of this rank's rows -> every rank's slots -> cur_stats[B][world][64]
 // B == 0: the signal / wait step alone -- the completion barrier of a layout switch that a GEMM's epilogue performed (its TMA stores to
 // the peers are complete when that kernel ends; this kernel, next in the stream, fences and publishes the sequence number).
-__global__ void __launch_bounds__(128) gn_peer_allreduce_kernel(const float* __restrict__ partial, int splits, int B, const __grid_constant__ PeerCommDev pc) {
-  const int tid = threadIdx.x;
-  float mine = 0.f;
-  if (tid < B * 64) {
-    const int b = tid >> 6, t = tid & 63;
-    for (int sp = 0; sp < splits; ++sp) mine += partial[((long long)b * splits + sp) * 64 + t];
-  }
-  peer_finish(pc, B, B > 0, mine, tid);
+__global__ void __launch_bounds__(PEER_ALLREDUCE_THREADS) gn_peer_allreduce_kernel(const float* __restrict__ partial, int splits, int B,
+                                                                                const __grid_constant__ PeerCommDev pc) {
+  peer_finish(pc, B, B > 0, partial, splits, threadIdx.x);
 }
 
 }  // namespace vc
@@ -212,7 +211,8 @@ int groupnorm_stats_partials(const __half* x1, int C1, int samples, long long ro
 
 static int to_dev(const vc_peer_comm* c, PeerCommDev& d) {
   VC_REQUIRE(c && c->world >= 1 && c->world <= PEER_MAX && c->rank >= 0 && c->rank < c->world, "peer comm: bad world / rank");
-  VC_REQUIRE(c->flags && c->seq && c->done && c->cur_stats && c->Bmax >= 1 && c->Bmax <= 2, "peer comm: null buffer or Bmax not in 1..2");
+  VC_REQUIRE(c->flags && c->seq && c->done && c->cur_stats && c->Bmax >= 1 && c->Bmax <= PEER_BMAX,
+             "peer comm: null buffer or Bmax not in 1..%d", PEER_BMAX);
   d.world = c->world; d.rank = c->rank;
   d.flags = reinterpret_cast<unsigned int*>(c->flags);
   d.seq = reinterpret_cast<unsigned int*>(c->seq);
@@ -308,6 +308,8 @@ int vc_peer_exchange(const vc_peer_comm* c, const void* src, void* const* dst, i
   p.rows_per_split = (p.rows_local + splits - 1) / splits;
   p.partial = reinterpret_cast<float*>(ws);
   VC_REQUIRE(!p.with_stats || (ws && ws_bytes >= (size_t)B * splits * 64 * sizeof(float)), "peer_exchange: workspace too small");
+  // the last CTA runs peer_finish: its threads loop over the B*64 sums, and one thread per rank signals / waits
+  VC_REQUIRE(p.vecs * p.ppi >= c->world && B <= PEER_BMAX, "peer_exchange: block of %d threads for world %d, B %d", p.vecs * p.ppi, c->world, B);
   dim3 grid(splits, B);
   peer_exchange_kernel<<<grid, p.vecs * p.ppi, p.with_stats ? (size_t)2 * C * p.ppi * sizeof(float) : 0, reinterpret_cast<cudaStream_t>(stream)>>>(p);
   VC_CHECK_CUDA(cudaGetLastError());
@@ -325,7 +327,7 @@ int vc_peer_groupnorm_stats(const vc_peer_comm* c, const void* x, int32_t C, int
   rc = groupnorm_stats_partials(reinterpret_cast<const __half*>(x), C, samples, rows_per_sample, reinterpret_cast<float*>(ws), ws_bytes,
                                 &splits, reinterpret_cast<cudaStream_t>(stream));
   if (rc) return rc;
-  gn_peer_allreduce_kernel<<<1, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float*>(ws), splits, samples, d);
+  gn_peer_allreduce_kernel<<<1, PEER_ALLREDUCE_THREADS, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float*>(ws), splits, samples, d);
   VC_CHECK_CUDA(cudaGetLastError());
   return VC_OK;
 }
@@ -349,7 +351,7 @@ int vc_peer_finish_scatter(const vc_peer_comm* c, const vc_gn_part_geom* geom, i
     if (rc) return rc;
     B = samples;
   }
-  gn_peer_allreduce_kernel<<<1, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float*>(ws), splits, B, d);
+  gn_peer_allreduce_kernel<<<1, PEER_ALLREDUCE_THREADS, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float*>(ws), splits, B, d);
   VC_CHECK_CUDA(cudaGetLastError());
   return VC_OK;
 }

@@ -144,16 +144,19 @@ class DDIMSampler(object):
         the sampler passes the same dicts for all steps (ddim.py:150-160), and handing the U-Net the SAME context tensor
         each step lets it keep the cross-attention K/V projections (SURVEY.md App. C.1).  Also reports whether the
         c_concat entries of the two branches are the same tensors (utils/diffusion_utils.py:152-153)."""
-        ents = [(a, u) for k in c for a, u in zip(c[k], uc[k])]
-        sig = [(a, ops.tensor_version(a), u, ops.tensor_version(u)) for a, u in ents]
+        return self._stack_conditionings((c, uc))
+
+    def _stack_conditionings(self, conds):
+        """_stacked_conditioning for any number of conditioning dicts with the same keys (stacked in the given order)."""
+        sig = [(a, ops.tensor_version(a)) for k in conds[0] for ent in zip(*(d[k] for d in conds)) for a in ent]
         cached = getattr(self, "_cat_cache", None)
-        if cached is not None and len(cached[0]) == len(sig) and all(va is not None and vu is not None for _, va, _, vu in sig) and all(
-                a is a0 and va == va0 and u is u0 and vu == vu0 for (a, va, u, vu), (a0, va0, u0, vu0) in zip(sig, cached[0])):
-            return cached[1], cached[2]
-        cat = {k: [torch.cat([a, u], 0) for a, u in zip(c[k], uc[k])] for k in c}
-        same = all((a is u) or (a.shape == u.shape and bool(torch.equal(a, u))) for a, u in zip(c.get("c_concat", []), uc.get("c_concat", []))) \
-            if "c_concat" in c else False
-        self._cat_cache = (sig, cat, same)
+        if cached is not None and cached[0] == len(conds) and len(cached[1]) == len(sig) and all(v is not None for _, v in sig) and all(
+                a is a0 and v == v0 for (a, v), (a0, v0) in zip(sig, cached[1])):
+            return cached[2], cached[3]
+        cat = {k: [torch.cat(ent, 0) for ent in zip(*(d[k] for d in conds))] for k in conds[0]}
+        same = all(all((a is e[0]) or (a.shape == e[0].shape and bool(torch.equal(a, e[0]))) for a in e[1:])
+                   for e in zip(*(d.get("c_concat", []) for d in conds))) if "c_concat" in conds[0] else False
+        self._cat_cache = (len(conds), sig, cat, same)
         return cat, same
 
     def _apply_both(self, x, t, c, uc, kwargs):

@@ -145,10 +145,11 @@ class PeerFrameComm(FrameComm):
       * to_sites / to_frames are ONE kernel each (rows stored straight into the owning rank's buffer; no pack / unpack copy),
       * the statistics of the 5-D GroupNorm that follows every to_sites ride along with it (no statistics pass, no all-reduce),
       * the GroupNorms in the middle of a temporal block exchange 2 x 32 floats per sample through the same flag protocol.
+    Up to `bmax` (<= 4) batch samples per rank: the three branches of three-way guidance run as one B=3 forward.
     The receive buffers are reused by every switch (one per direction): tensors returned by to_sites()/to_frames() are views
     of them and are only valid until the next switch in the same direction -- UNetModel clones the ones it keeps as skips."""
 
-    def __init__(self, dist, rank: int, world: int, group, device, bmax: int = 2):
+    def __init__(self, dist, rank: int, world: int, group, device, bmax: int = 4):
         super().__init__(dist, rank, world, group)
         from . import _lib
         self.lib = _lib.load()
@@ -368,6 +369,17 @@ class CfgComm:
         buf = v_mine.new_empty((2, *v_mine.shape))
         self.dist.all_gather_into_tensor(buf.view(-1), v_mine.contiguous().view(-1), group=self.pair_group)   # pair group rank order = (cond, uncond)
         return buf[0], buf[1]
+
+    def exchange3(self, v_a: torch.Tensor, v_b: torch.Tensor = None):
+        """Three-way guidance: branch 0 passes (v_cond, v_img), branch 1 passes v_uncond (its second slot is padding); one all-gather
+        of a 2-slot buffer per pair.  Returns (v_cond, v_uncond, v_img) on every rank."""
+        mine = v_a.new_zeros((2, *v_a.shape))
+        mine[0] = v_a
+        if v_b is not None:
+            mine[1] = v_b
+        buf = v_a.new_empty((2, 2, *v_a.shape))
+        self.dist.all_gather_into_tensor(buf.view(-1), mine.view(-1), group=self.pair_group)
+        return buf[0, 0], buf[1, 0], buf[0, 1]
 
 
 def _make_comm(dist, rank, world, group, device, peer: bool):

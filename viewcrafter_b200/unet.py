@@ -41,6 +41,11 @@ def _ln_linear(Q: dict, x: torch.Tensor, name: str, ln: str, st=None, **kw) -> t
     return ops.linear(ops.layernorm(x, *Q[ln]), Q[name], bias=Q[name + "_b"], **kw)
 
 
+# cfg_shared_prefix=True asks for the shared CFG prefix on one GPU only: the two-way sampler sends it to frame-sharded forwards too, which
+# run the plain B=2 path.  This value asks for it under frame sharding as well (the three-way sampler's stacked calls).
+SHARED_PREFIX_ANY_LAYOUT = "any_layout"
+
+
 def _unsupported(flag: str):
     raise NotImplementedError(f"viewcrafter_b200.UNetModel: option {flag} is not on the ViewCrafter inference path")
 
@@ -397,9 +402,9 @@ class UNetModel(nn.Module):
 
     @staticmethod
     def _spatial_tf(P, h, ctx, B, T, H, W, expand=False, out_plan=None):
-        """expand=True (shared CFG prefix, SURVEY.md App. C.2): `h` holds ONE batch element that is identical for the B=2
-        conditional / unconditional branches; everything up to and including attn1 of the first block does not see the
-        context, so it runs once and is duplicated right before the first cross-attention."""
+        """expand=True (shared CFG prefix, SURVEY.md App. C.2): `h` holds ONE batch element that is identical for the B (2 or 3)
+        guidance branches; everything up to and including attn1 of the first block does not see the context, so it runs once
+        and is replicated to B rows right before the first cross-attention."""
         Bc = 1 if expand else B
         BT, HW, heads = Bc * T, H * W, P["heads"]
         C = heads * 64
@@ -412,8 +417,8 @@ class UNetModel(nn.Module):
             x = ops.linear(a, Q["o1_w"], bias=Q["o1_b"], res=x, ln_out=fold)
             x, st = x if fold else (x, None)
             if expand:
-                x, h = torch.cat([x, x], 0), torch.cat([h, h], 0)
-                st = torch.cat([st, st], 0) if st is not None else None
+                x, h = torch.cat([x] * B, 0), torch.cat([h] * B, 0)
+                st = torch.cat([st] * B, 0) if st is not None else None
                 expand, Bc, BT = False, B, B * T
             q = _ln_linear(Q, x, "q2", "ln2", st)
             a = torch.empty_like(q)
@@ -463,17 +468,21 @@ class UNetModel(nn.Module):
         out = ops.linear(x, P["out_w"], bias=P["out_b"], res=t_in, gn_out=comm is None, peer=to_f)
         return out if to_f is not None else (comm.to_frames(out, B, HW) if comm else out)
 
-    def _run_stage(self, stage, h, skip, emb, ctx, B, T, H, W):
+    def _run_stage(self, stage, h, skip, emb, ctx, B, T, H, W, emb1=None):
+        """emb1 (shared CFG prefix): `h` holds ONE batch element common to the B branches; the ResBlock before the first
+        SpatialTransformer runs on it with emb1 (the branches' common embedding row) and that transformer expands to B rows."""
         comm, pre_sites = self._comm, False
+        Bc = 1 if emb1 is not None else B
         for idx, P in enumerate(stage):
             k = P["kind"]
             if k == "R":
-                h = self._res(P, h, skip, emb, B, T, H, W, comm)
+                h = self._res(P, h, skip, emb if Bc == B else emb1, Bc, T, H, W, comm)
                 skip = None
             elif k == "S":
                 nxt = stage[idx + 1]["kind"] if idx + 1 < len(stage) else None
                 plan = comm.scatter_plan(True, B, H * W, P["out_w"].shape[0]) if (comm and nxt == "T") else None
-                h = self._spatial_tf(P, h, ctx, B, T, H, W, out_plan=plan)
+                h = self._spatial_tf(P, h, ctx, B, T, H, W, expand=Bc != B, out_plan=plan)
+                Bc = B
                 pre_sites = plan is not None
             elif k == "T":
                 h = self._temporal_tf(P, h, B, T, H, W, comm, pre_sites=pre_sites)
@@ -553,7 +562,7 @@ class UNetModel(nn.Module):
 
     def _forward_graphed(self, x, timesteps, context, fs, kwargs):
         ver = ops.tensor_version(context)
-        flags = tuple(sorted((k, bool(v)) for k, v in kwargs.items() if k == "cfg_shared_prefix"))
+        flags = tuple(sorted((k, v if isinstance(v, str) else bool(v)) for k, v in kwargs.items() if k == "cfg_shared_prefix"))
         key = (tuple(x.shape), x.dtype, id(context), ver, fs is None, flags, id(self._comm))
         e = self._graphs.get(key)
         if ver is None or (e is not None and e["ctx"] is not context):
@@ -601,10 +610,11 @@ class UNetModel(nn.Module):
         B, Cin, T, H, W = x.shape
         dev = x.device
         x32 = x.float().contiguous()
-        # cfg_shared_prefix: the caller (DDIMSampler._apply_both) asserts that batch rows 0 and 1 carry the same x, t, fs
-        # and c_concat and differ only in the cross-attention context
+        # cfg_shared_prefix: the caller (DDIMSampler._apply_both, the three-way sampler) asserts that all B (2 or 3) batch rows carry the
+        # same x, t, fs and c_concat and differ only in the cross-attention context
         kinds = [Pm["kind"] for Pm in P["input"][1]] if len(P["input"]) > 1 else []
-        shared = bool(kwargs.get("cfg_shared_prefix")) and B == 2 and comm is None and kinds[:2] == ["R", "S"]
+        flag = kwargs.get("cfg_shared_prefix")
+        shared = bool(flag) and B in (2, 3) and (comm is None or flag == SHARED_PREFIX_ANY_LAYOUT) and kinds[:2] == ["R", "S"]
         # --- embeddings (fp32) : time_embed(t) + fps_embedding(fs), one row per batch element (frame-invariant) ---
         ts = timesteps.to(device=dev, dtype=torch.int64).contiguous()
         tw = P["time"]
@@ -629,32 +639,22 @@ class UNetModel(nn.Module):
         ops.ncthw_to_rows(x32, h, 0)
 
         hs = []
-        first = 0
+        emb1 = None
         if shared:
-            # SURVEY.md App. C.2: both CFG branches see the same x, t, fs and c_concat, so everything before the first
+            # SURVEY.md App. C.2: all guidance branches see the same x, t, fs and c_concat, so everything before the first
             # cross-attention (input_blocks.0, init_attn, input_blocks.1.0 and input_blocks.1.1 up to attn1) is computed once
-            # on one batch element and duplicated; the results are those of the plain B=2 forward.
+            # on one batch element and replicated to B rows; the results are those of the plain B-row forward.  Under frame
+            # sharding the prefix's layout switches run at B=1.
             emb1 = emb[:1].contiguous()
             h = h[:T * H * W]
             h, H, W = self._run_stage(P["input"][0], h, None, emb1, ctx, 1, T, H, W)
             if self.addition_attention:
                 h, H, W = self._run_stage(P["init_attn"], h, None, emb1, ctx, 1, T, H, W)
-            hs.append(torch.cat([h, h], 0))
-            Bc = 1
-            for Pm in P["input"][1]:
-                if Bc == 1 and Pm["kind"] == "R":
-                    h = self._res(Pm, h, None, emb1, 1, T, H, W, None)
-                elif Bc == 1 and Pm["kind"] == "S":
-                    h = self._spatial_tf(Pm, h, ctx, B, T, H, W, expand=True)
-                    Bc = B
-                else:
-                    h, H, W = self._run_stage([Pm], h, None, emb, ctx, B, T, H, W)
-            hs.append(h)
-            first = 2
+            hs.append(torch.cat([h] * B, 0))       # a copy: also detaches the skip from a reusable peer receive buffer
         for i, stage in enumerate(P["input"]):
-            if i < first:
+            if i == 0 and shared:
                 continue
-            h, H, W = self._run_stage(stage, h, None, emb, ctx, B, T, H, W)
+            h, H, W = self._run_stage(stage, h, None, emb, ctx, B, T, H, W, emb1=emb1 if i == 1 else None)
             if i == 0 and self.addition_attention:
                 h, H, W = self._run_stage(P["init_attn"], h, None, emb, ctx, B, T, H, W)
             if comm and getattr(comm, "owns", None) and comm.owns(h):
