@@ -403,7 +403,13 @@ def shard_model(model, dist, rank: int, world: int, cfg_split: bool = True, peer
 
     world even and cfg_split: 2-way CFG split x (world/2)-way frame sharding -- e.g. 8 GPUs = 2 x 4 with frames 7/6/6/6
     (ideal 7.1x) instead of 8-way frames 4/3x7 (ideal 6.25x).  Otherwise pure frame sharding.
-    Every rank must call this (it creates process groups collectively).  Returns the FrameComm (or None)."""
+    Every rank must call this (it creates process groups collectively).  Returns the FrameComm (or None).
+
+    A model with a ``first_stage_model`` also gets ``model._vae``: a FrameComm over the whole world, which makes
+    ``synthesis.get_latent_z`` and the decode of ``synthesis.image_guided_synthesis`` split their per-frame VAE work over all
+    ranks (vae_encode_sharded / vae_decode_sharded)."""
+    if world > 1 and getattr(model, "first_stage_model", None) is not None:
+        model._vae = FrameComm(dist, rank, world, None)          # the VAE has no CFG branches: all ranks share its frames
     unet = model.model.diffusion_model if hasattr(model, "model") else model
     try:
         device = next(unet.parameters()).device
@@ -422,3 +428,57 @@ def shard_model(model, dist, rank: int, world: int, cfg_split: bool = True, peer
         return unet._comm
     unet._comm = _make_comm(dist, rank, world, None, device, peer)
     return unet._comm
+
+
+# -- the VAE stages of a clip ------------------------------------------------------------------------------------------------------
+# The VAE works on one frame at a time (per-frame GroupNorm, one single-image AttnBlock per frame), so its work splits by frame with
+# no communication inside it: rank r runs its frame range of every sample, then the results are all-gathered (FrameComm.gather_frames).
+# Only attributes the reference's VIPLatentDiffusion also has are used (first_stage_model.encode, get_first_stage_encoding,
+# decode_first_stage, perframe_ae), so the reference model with the viewcrafter_b200 networks swapped in is sharded the same way.
+
+def vae_encode_sharded(model, videos: torch.Tensor) -> torch.Tensor:
+    """videos [b, c, T, H, W] -> latents [b, c', T, H/8, W/8] on every rank, equal to what get_latent_z returns in one process.
+
+    Rank r encodes frames [t0, t1) of every sample (one call per frame when perframe_ae, else one call) and keeps the posterior
+    moments; the moments are all-gathered, and every rank then draws the posterior samples itself in the reference's order
+    (ddpm3d.py:620-644: one draw per frame in (b t) order when perframe_ae, else one draw over all frames).  So every rank consumes
+    the CPU generator exactly as a single process does and ends in its state: x_T, the per-step noise and the next clip's draws
+    stay the reference's.  (Calling encode_first_stage on a frame slice would draw the noise of the wrong frames.)"""
+    from .distributions import posterior_class
+    comm = model._vae
+    b, c, T, H, W = videos.shape
+    t0, t1 = comm.bind(T)
+    vae = model.first_stage_model
+    if t1 > t0:
+        x = videos[:, :, t0:t1].permute(0, 2, 1, 3, 4).reshape(b * (t1 - t0), c, H, W)
+        posts = [vae.encode(x[i:i + 1]) for i in range(x.shape[0])] if model.perframe_ae else [vae.encode(x)]
+        cls = type(posts[0])                        # the reference's own posterior class when its AutoencoderKL is used
+        m = torch.cat([p.parameters for p in posts], 0)
+        local = m.reshape(b, t1 - t0, *m.shape[1:]).permute(0, 2, 1, 3, 4)
+    else:
+        # T < world: no frames here, only the gather padding.  The fp32 moments and the posterior class are what
+        # viewcrafter_b200's AutoencoderKL.encode returns (posterior_class() subclasses the reference's class when that is loaded).
+        f = 2 ** (len(vae.encoder.down) - 1)
+        local = videos.new_empty((b, 2 * vae.embed_dim, 0, H // f, W // f), dtype=torch.float32)
+        cls = posterior_class()
+    moments = comm.gather_frames(local, T).permute(0, 2, 1, 3, 4).flatten(0, 1)      # [(b T), 2*embed, h, w]
+    if model.perframe_ae:
+        z = torch.cat([model.get_first_stage_encoding(cls(moments[i:i + 1])).detach() for i in range(b * T)], 0)
+    else:
+        z = model.get_first_stage_encoding(cls(moments)).detach()
+    return z.reshape(b, T, *z.shape[1:]).permute(0, 2, 1, 3, 4)
+
+
+def vae_decode_sharded(model, samples: torch.Tensor) -> torch.Tensor:
+    """latents [b, c, T, h, w] -> the decoded video [b, out_ch, T, 8h, 8w] on every rank: rank r decodes frames [t0, t1) through
+    the model's own decode_first_stage (so its perframe_ae / decode_batch rules apply to the slice), then the frames are gathered."""
+    comm = model._vae
+    b, _, T, h, w = samples.shape
+    t0, t1 = comm.bind(T)
+    if t1 > t0:
+        local = model.decode_first_stage(samples[:, :, t0:t1])
+    else:                                                                      # T < world: only the gather padding
+        dec = model.first_stage_model.decoder
+        f = 2 ** (len(dec.up) - 1)
+        local = samples.new_empty((b, dec.conv_out.out_channels, 0, h * f, w * f))
+    return comm.gather_frames(local, T)

@@ -13,18 +13,24 @@ What differs from the reference, all parity-preserving (SURVEY.md App. C):
     iteration -- the cross-attention K/V projections are computed once per clip;
   * ``cuda_graph=True`` lets the viewcrafter_b200 U-Net replay its forward as one captured CUDA graph from the third call on
     (``UNetModel.enable_cuda_graph``): same kernels in the same order, ~1000 launches -> 1 per forward;
+  * under ``parallel.shard_model`` the VAE encode and decode are split by frame over all ranks (``parallel.vae_encode_sharded`` /
+    ``vae_decode_sharded``), with the posterior draws still taken in the reference's order on every rank;
   * nothing else: conditioning tensors, ``x_T`` / per-step noise draws and the decode are the reference's, in its order.
 """
 from __future__ import annotations
 
 import torch
 
+from . import parallel
 from .ddim import DDIMSampler
 from .ddim_multiplecond import DDIMSampler as DDIMSampler_multicond
 
 
 def get_latent_z(model, videos):
-    """videos [b, c, t, h, w] -> latents [b, c', t, h/8, w/8] via per-frame encode_first_stage (diffusion_utils.py:110-115)."""
+    """videos [b, c, t, h, w] -> latents [b, c', t, h/8, w/8] via per-frame encode_first_stage (diffusion_utils.py:110-115).
+    Under parallel.shard_model the frames are encoded on all ranks (parallel.vae_encode_sharded): same result, same RNG draws."""
+    if getattr(model, "_vae", None) is not None:
+        return parallel.vae_encode_sharded(model, videos)
     b, c, t, h, w = videos.shape
     x = videos.permute(0, 2, 1, 3, 4).reshape(b * t, c, h, w)
     z = model.encode_first_stage(x)
@@ -84,5 +90,7 @@ def image_guided_synthesis(model, prompts, videos, noise_shape, n_samples=1, ddi
                                          unconditional_guidance_scale=unconditional_guidance_scale, unconditional_conditioning=uc,
                                          eta=ddim_eta, cfg_img=cfg_img, mask=None, x0=None, fs=fs,
                                          timestep_spacing=timestep_spacing, guidance_rescale=guidance_rescale, **kwargs)
-        batch_variants.append(model.decode_first_stage(samples))             # latent -> pixel space
+        # latent -> pixel space; under parallel.shard_model every rank decodes its frames and gathers the rest
+        sharded = getattr(model, "_vae", None) is not None
+        batch_variants.append(parallel.vae_decode_sharded(model, samples) if sharded else model.decode_first_stage(samples))
     return torch.stack(batch_variants).permute(1, 0, 2, 3, 4, 5)              # batch, variants, c, t, h, w
